@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (CUDA, through the C ABI)
   python bench.py --impl reference ...                            # the reference's CPU path, restated (oracle port)
+  python bench.py ... --dump-outputs DIR                          # + the last timed step's decisions as DIR/*.npy
 
 Step      one pass of the hot path over one wave: the request phase of 65 536 non-streaming chat requests
           (1 KiB bodies, 10 000 tenants, Qwen-style chat JSON) followed by the response phase of every admitted
@@ -24,11 +25,13 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; nothing is written into it
 
 import numpy as np  # noqa: E402
 
@@ -58,7 +61,13 @@ def parse_args():
     ap.add_argument("--fold-every", type=int, default=8)
     ap.add_argument("--latency-requests", type=int, default=10_000_000,
                     help="requests per GPU in the 1.25 M/s open-loop latency run (SURVEY.md section 8d: >= 10 M; 8 s of arrivals)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the decisions of the last timed step (rank 0) as DIR/request_<field>.npy and DIR/response_<field>.npy "
+                         "(float64); the inputs are seeded, so two builds run with the same arguments can be compared array by array")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return a
 
 
 def env_rank():
@@ -122,7 +131,7 @@ def bpe_section(g, w, reqs, resps, now, peak, ext, sample=2048):
     size (151 k merges) trained with `tokenizers` on synthetic text, same pre-tokenizer and algorithm."""
     from arks_b200 import bpe
     t0 = time.perf_counter()
-    tok, text = bpe.standin_tokenizer(151_643, cache_dir=os.path.join(ROOT, "tests", "_build"))
+    tok, text = bpe.standin_tokenizer(151_643)
     tables = bpe.load_tokenizer(text)
     vocab_s = time.perf_counter() - t0
     import torch
@@ -168,6 +177,9 @@ def bpe_section(g, w, reqs, resps, now, peak, ext, sample=2048):
     # the sample: first `sample` rows of wave 0 against `tokenizers`, and through the host build for the table probes
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import hostmachine as hm
+    with tempfile.TemporaryDirectory() as tmp:
+        hm.OUT = os.path.join(tmp, os.path.basename(hm.OUT))  # compiled for this run, outside the tree
+        hm.lib()
     hm.bpe_load(tables)
     hm.bpe_probes()
     rb = reqs[0]
@@ -241,6 +253,20 @@ def pin_batch(b):
         setattr(b, name, t.numpy())
         b.__dict__.setdefault("_pins", []).append(t)
     return b
+
+
+def write_outputs(out_dir, dump, cap=60 << 20):
+    """The decision arrays a caller of the timed path receives, as float64 (every value is an integer below 2**53):
+    request_<field>.npy and response_<field>.npy, one row per request / response (usage: 3 columns). <phase>_row.npy holds
+    the row numbers: every row while the arrays fit in `cap` bytes, else the same seeded sample of rows on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    phases = {p: {"row": np.arange(len(dump[p].reason)), **dump[p].fields()} for p in ("request", "response")}
+    total = sum(8 * a.size for f in phases.values() for a in f.values())
+    for phase, f in phases.items():
+        n = len(f["row"])
+        keep = np.arange(n) if total <= cap else np.sort(np.random.default_rng(0).choice(n, n * cap // total, replace=False))
+        for name, a in f.items():
+            np.save(os.path.join(out_dir, f"{phase}_{name}.npy"), a[keep].astype(np.float64))
 
 
 def peaks():
@@ -484,11 +510,19 @@ def run_b200(args):
     torch.cuda.synchronize()
 
     fold_events, fold_host_us = [], []
+    dump = {} if args.dump_outputs and rank == 0 else None
 
-    def resident_step(i, now, fold=True):
+    def resident_step(i, now, fold=True, keep=None):
         k = i % N_WAVES
         g.select_slot(k)
         g.run_request(now)
+        if keep is not None:
+            # the response phase writes its decisions over the request phase's on the device: copy those out first, between
+            # two events, so that the copy can be taken out of the timed region
+            keep["events"] = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            keep["events"][0].record(ext)
+            keep["request"] = g.fetch_request(reqs[k].n)
+            keep["events"][1].record(ext)
         g.run_response(now + 1)
         if fold and args.shared_quota and i % args.fold_every == args.fold_every - 1:
             # stream-ordered behind this step's kernels; nobody waits on the host. Timed on both sides: the device time includes
@@ -506,11 +540,14 @@ def run_b200(args):
         now += STEP_S
     sampler = ClockSampler(local)
     sampler.start()
-    # keep the GPU under this workload until nvidia-smi has produced its first samples
+    # keep the GPU under this workload until nvidia-smi has produced its first samples. A wall-clock loop: its length differs
+    # per rank (a collective inside would not pair up) and per run, so it runs request phases only. Those bill no quota, and
+    # every step opens fresh rate windows, so the timed steps below start from the same counters however long this took.
     t_spin = time.perf_counter()
     i = 0
     while time.perf_counter() - t_spin < 0.6:
-        resident_step(i, now, fold=False)  # a wall-clock loop: its length differs per rank, a collective inside would not pair up
+        g.select_slot(i % N_WAVES)
+        g.run_request(now)
         now += STEP_S
         i += 1
     barrier()
@@ -518,12 +555,16 @@ def run_b200(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(ext)
     for i in range(args.steps):
-        resident_step(args.warmup + i, now)
+        resident_step(args.warmup + i, now, keep=dump if i == args.steps - 1 else None)
         now += STEP_S
     e1.record(ext)
     barrier()
     launches = g.launch_count - launches0
     dev_ms = e0.elapsed_time(e1)
+    if dump is not None:
+        dev_ms -= dump["events"][0].elapsed_time(dump["events"][1])
+        dump["response"] = g.fetch_response(resps[(args.warmup + args.steps - 1) % N_WAVES].n)
+        write_outputs(args.dump_outputs, dump)
     shared_quota = None
     if args.shared_quota:
         # one fold epoch timed alone (gather + all-reduce + apply), every rank in step
